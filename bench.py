@@ -17,6 +17,9 @@ no data-path collective inside Hψ; the density allreduce of an SCF step is time
 `roofline_gemm` = the nonlocal P D P†ψ GEMMs (FP64 DMMA; 16·N_pw·n_proj·M flop) against a cuBLAS ZGEMM
              probe measured in the same run (MEASURED_PEAKS.json has no FP64 figure).
 `cpu_baseline` = the CPU oracle (port of the reference's band-at-a-time algorithm) on a bounded sample.
+
+`--dump-outputs DIR` writes Hψ of the last timed step to DIR/hpsi.npy so that two builds can be compared output for output:
+ψ and the operator depend only on the arguments (seeded generator), so the same arguments give the same inputs.
 """
 import argparse
 import json
@@ -87,6 +90,22 @@ def peaks():
         d = json.load(open(p))
         return d.get("hbm_gbs", 6650.0), "MEASURED_PEAKS.json hbm_gbs (driver-measured copy bandwidth)"
     return 6650.0, "fallback 6.65 TB/s (B200_PROFILING.md)"
+
+
+DUMP_BYTES = 32 << 20       # all ranks together; a larger Hψ is sampled
+
+
+def dump_outputs(path, torch, hpsi, rank, world):
+    """Save Hψ (M x n_pw complex) as float64 (n, 2) = (real, imag) rows of the band-major flattened array: all of it when
+    it fits DUMP_BYTES / world, else the same seeded sample of entries (seed 0, increasing order) on every run.  Rank r > 0
+    of a multi-GPU run writes hpsi_rank<r>.npy."""
+    os.makedirs(path, exist_ok=True)
+    flat = torch.view_as_real(hpsi).reshape(-1, 2)
+    n_keep = min(flat.shape[0], DUMP_BYTES // world // 16)
+    if n_keep < flat.shape[0]:
+        idx = np.sort(np.random.default_rng(0).choice(flat.shape[0], n_keep, replace=False))
+        flat = flat[torch.from_numpy(idx).to(flat.device)]
+    np.save(os.path.join(path, "hpsi.npy" if rank == 0 else f"hpsi_rank{rank}.npy"), flat.cpu().numpy())
 
 
 class ClockSampler:
@@ -388,6 +407,8 @@ def run_gpu(args):
     clocks = sampler.stop() if sampler else None
     ms_step = ms_total / args.steps
     value = world * M * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs:           # before the sections below overwrite hpsi
+        dump_outputs(args.dump_outputs, torch, hpsi, rank, world)
 
     # ---- kernel-group breakdown (same stream, CUDA events)
     ms_local = timed(lambda: kb.apply_terms(psi, 3, out=hpsi), max(2, args.steps // 2), 1) / max(2, args.steps // 2)
@@ -737,7 +758,13 @@ def main():
     ap.add_argument("--slab-scf-steps", type=int, default=0, help="SCF iterations of the single-k slab section when --scf-steps is 0")
     ap.add_argument("--scf-tol", type=float, default=0.025)
     ap.add_argument("--scf-maxiter", type=int, default=6)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write H psi of the last timed step to DIR/hpsi.npy (float64 real/imag pairs, seeded sample when large)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
     if args.cpu_bands <= 0:
         args.cpu_bands = 64      # enough columns for the CPU ZGEMM not to be bound by the bandwidth of P
